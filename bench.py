@@ -6,6 +6,7 @@ quoted on); --config 3 | 4 | 5 selects the other BASELINE configurations.
     python bench.py --gpus 1 --steps K --warmup W             engine arm (this repo's CUDA engine)
     python bench.py --impl reference --gpus N --steps K ...    reference arm: the reference's PyTorch path on the host
                                                                cores (oracle/ref_path.py driving torch CPU ops)
+    python bench.py ... --dump-outputs DIR                     also write the last timed step's z and losses as DIR/*.npy
 
 One "step" = one train() iteration (pixray.py:1436-1512): synth -> MakeCutouts -> encode_image -> Prompt losses ->
 backward -> Adam -> clip_z.  Prints ONE JSON line on rank 0.
@@ -350,6 +351,8 @@ def run_engine(args, cfg, rank, world):
     sampler.stop_flag = True
     ms = e0.elapsed_time(e1)
     launches = eng.num_launches() - n0
+    if args.dump_outputs and rank == 0:  # before profile_iteration, which steps z once more
+        dump_outputs(args.dump_outputs, z=z, losses=eng.read_losses())
     # ---- per-kernel split for the roofline of the dominant kernel family
     prof = eng.profile_iteration(z, lr, args.warmup + args.steps)
     barrier()
@@ -454,6 +457,16 @@ def run_engine(args, cfg, rank, world):
         dist.destroy_process_group()
 
 
+def dump_outputs(out_dir, **arrays):
+    """--dump-outputs: what a caller of the timed path holds after its last step (z, updated in place, and the loss vector
+    of that step), one float32 DIR/<name>.npy each.  z is at most a few MB in every config, so it is written whole.
+    Measured on a B200: two runs of config 2 give identical bits; configs 4 (vdiff) and 5 (fft) do not, on identical inputs."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if torch.is_tensor(a) else np.asarray(a)
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.astype(np.float32))
+
+
 _JSON_FD = None
 
 
@@ -482,7 +495,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--parallel", default="shard", choices=["shard", "replicas"],
                     help="N > 1: shard the cutouts of one problem over the ranks (default) or run N independent replicas")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last timed step's outputs (z, losses) as DIR/<name>.npy; the "
+                         "inputs are seeded, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "engine":
+        ap.error("--dump-outputs dumps the engine arm's timed path")
     if args.warmup < 3:
         args.warmup = 3
     cfg = CONFIGS[args.config]

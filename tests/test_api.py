@@ -312,13 +312,10 @@ def test_file_image_prompts_keep_their_aspect_ratio(fake, tmp_path):
 
 def test_spot_prompts_reach_the_engine(fake, tmp_path):
     """args.spot_prompts / spot_prompts_off (pixray.py:917-931) with the reference's own mask image (inputs/spot_square.png,
-    fetch_spot_indexes pixray.py:370-394) resized to the cut size."""
-    ref_inputs = "/root/reference/inputs/spot_square.png"
-    if not os.path.exists(ref_inputs):
-        pytest.skip("reference checkout not present")
+    stored as tests/golden/spot_square.png; fetch_spot_indexes pixray.py:370-394) resized to the cut size."""
     (tmp_path / "inputs").mkdir(exist_ok=True)
     import shutil
-    shutil.copy(ref_inputs, tmp_path / "inputs" / "spot_square.png")
+    shutil.copy(os.path.join(os.path.dirname(__file__), "golden", "spot_square.png"), tmp_path / "inputs" / "spot_square.png")
     _init(tmp_path, prompts="x", clip_models="ViT-B/32,ViT-B/16", spot_prompts="a red circle:2|a dot", spot_prompts_off="the sky")
     eng = api._state.engine
     calls = [c for c in eng.calls if c[0] == "set_spot_prompts"]
