@@ -33,6 +33,8 @@ typedef struct pxr_engine* pxr_handle;
 enum { PXR_DRAWER_VQGAN = 0, PXR_DRAWER_PIXEL = 1, PXR_DRAWER_FFT = 2, PXR_DRAWER_VDIFF = 3 };
 enum { PXR_PAD_REFLECTION = 0, PXR_PAD_BORDER = 1, PXR_PAD_ZEROS = 2 };
 enum { PXR_DTYPE_F16 = 0, PXR_DTYPE_BF16 = 1 };
+/* optimiser kinds for pxr_set_optimizer (args.optimiser, pixray.py:536-553; library defaults, only lr is set) */
+enum { PXR_OPT_ADAM = 0, PXR_OPT_ADAMW = 1, PXR_OPT_ADAGRAD = 2, PXR_OPT_ADAMAX = 3, PXR_OPT_DIFFGRAD = 4 };
 /* module ids for pxr_load_weight */
 enum { PXR_MOD_VQGAN = 0, PXR_MOD_CLIP0 = 1, PXR_MOD_CLIP1 = 2 };
 
@@ -211,7 +213,10 @@ int pxr_vdiff_set_clip_embed(pxr_handle h, const float* embed, int D);
 int pxr_vdiff_set_iteration(pxr_handle h, int i);
 int pxr_vdiff_renoise(pxr_handle h, float* z, int i, const float* noise);
 
-int pxr_reset_optimizer(pxr_handle h); /* rebuild_optimisers: fresh Adam state (pixray.py:520-555, 1511) */
+int pxr_reset_optimizer(pxr_handle h); /* rebuild_optimisers: fresh state of the current optimiser (pixray.py:520-555, 1511) */
+/* rebuild_optimisers with another args.optimiser: selects PXR_OPT_* `kind` (Adam after pxr_create), then does exactly
+ * what pxr_reset_optimizer does.  Every later pxr_step / pxr_iterate steps that optimiser. */
+int pxr_set_optimizer(pxr_handle h, int kind);
 
 /* train()'s control decisions on the device (checkdrop pixray.py:1090-1109; scheduled learning-rate drops, auto-stop and
  * rebuild_optimisers 1464-1512): the optimiser step of every pxr_iterate reads the iteration's loss vector, tracks the best
@@ -240,10 +245,12 @@ int pxr_set_batches(pxr_handle h, int batches);
 int pxr_set_z_grad(pxr_handle h, const float* z_grad);
 int pxr_sync(pxr_handle h);
 
-/* Checkpoint of the optimisation state for resume (SURVEY.md 8f-3): {z, Adam m, v, step count, learning-rate / best-loss /
- * drop bookkeeping} as one host blob of pxr_state_size bytes.  Load into an engine of the same configuration (after
- * pxr_set_schedule when the saved session was device-managed) and keep calling pxr_iterate with the next iteration number:
- * the engine-drawn augmentations are keyed by (seed, iteration), so the continuation follows the uninterrupted run. */
+/* Checkpoint of the optimisation state for resume (SURVEY.md 8f-3): {z, optimiser state m, v (+ DiffGrad's previous
+ * gradient), optimiser kind, step count, learning-rate / best-loss / drop bookkeeping} as one host blob of pxr_state_size
+ * bytes (the size depends on the current optimiser kind).  Load into an engine of the same configuration and optimiser
+ * kind (after pxr_set_schedule when the saved session was device-managed) and keep calling pxr_iterate with the next
+ * iteration number: the engine-drawn augmentations are keyed by (seed, iteration), so the continuation follows the
+ * uninterrupted run. */
 int pxr_state_size(pxr_handle h, int64_t* nbytes);
 int pxr_save_state(pxr_handle h, void* host_buf);
 int pxr_load_state(pxr_handle h, const void* host_buf);

@@ -66,7 +66,7 @@ class TestGemmDesc(C.Structure):
 EXPORTS = [
     "pxr_last_error", "pxr_version", "pxr_create", "pxr_destroy", "pxr_load_weight", "pxr_finalize",
     "pxr_set_prompts", "pxr_set_comm", "pxr_get_unique_id", "pxr_synth", "pxr_vqgan_encode", "pxr_make_cutouts", "pxr_encode_image",
-    "pxr_prompt_loss", "pxr_backward", "pxr_step", "pxr_iterate", "pxr_reset_optimizer", "pxr_sync",
+    "pxr_prompt_loss", "pxr_backward", "pxr_step", "pxr_iterate", "pxr_reset_optimizer", "pxr_set_optimizer", "pxr_sync",
     "pxr_num_kernel_launches", "pxr_get_stream", "pxr_z_numel", "pxr_z_bounds", "pxr_test_gemm", "pxr_test_conv", "pxr_debug_read", "pxr_profile_iteration", "pxr_profile_iteration2",
     "pxr_test_attention", "pxr_test_color_jitter_host", "pxr_test_color_jitter_device", "pxr_set_color_jitter", "pxr_set_image_prompts", "pxr_set_image_prompts_sized", "pxr_add_aux_loss", "pxr_add_filter", "pxr_clear_filters", "pxr_set_filter_shifts", "pxr_clear_aux_losses", "pxr_add_anchor", "pxr_clear_anchors", "pxr_num_losses", "pxr_read_losses",
     "pxr_test_pool_bounds", "pxr_test_groupnorm", "pxr_set_spot_prompts", "pxr_set_spot_mask", "pxr_state_size", "pxr_save_state", "pxr_load_state", "pxr_set_schedule", "pxr_poll_status", "pxr_set_batches", "pxr_set_z_grad", "pxr_vdiff_set_schedule", "pxr_vdiff_set_clip_embed", "pxr_vdiff_set_iteration", "pxr_vdiff_renoise",
@@ -98,5 +98,7 @@ def load():
             fn.restype = C.c_int
     if hasattr(lib, "pxr_last_error"):
         lib.pxr_last_error.argtypes = [C.c_void_p]
+    if hasattr(lib, "pxr_set_optimizer"):
+        lib.pxr_set_optimizer.argtypes = [C.c_void_p, C.c_int]
     _lib = lib
     return lib

@@ -5,8 +5,9 @@ front-ends use (run.py, cogrun.py) plus the notebook one-liner.
 Scope (SURVEY.md 8): the per-iteration hot path.  Every option of the reference's parser is KNOWN here (same dest,
 same default: the "requested setting not found" check of pixray.py:2088-2093 behaves identically), but options that
 switch on something outside the hot path (spot prompts, overlays, animation, init images through the VQGAN encoder,
-filters, transparency, non-Adam optimisers, SLIP perceptors, video) raise NotImplementedError when they are set to a
-non-default value instead of being silently ignored.  What the reference fetches from the network at init time comes in
+filters, transparency, the AdamP optimiser, SLIP perceptors, video) raise NotImplementedError when they are set to a
+non-default value instead of being silently ignored.  `optimiser` takes Adam, AdamW, Adagrad, Adamax or DiffGrad, each
+with its library's defaults like the reference builds them (pixray.py:536-553).  What the reference fetches from the network at init time comes in
 through three extra settings instead:
 
     b200_weights        {"vqgan": state_dict | path, "ViT-B/16": state_dict | path, ...} with the reference's own keys
@@ -107,7 +108,7 @@ _ENGINE_OPTIONS = [(("--b200_weights",), "b200_weights", None, None), (("--b200_
 _OFF_PATH = {
     "labels": ([],),
     "target_images": (None, []), "animation_dir": (None,),
-    "perceptors": ("clip",), "optimiser": ("Adam",), "make_video": (False,), "transparent": (False,),
+    "perceptors": ("clip",), "optimiser": tuple(E.OPTIMISERS), "make_video": (False,), "transparent": (False,),
     "image_prompt_shuffle": (False,),
 }
 
@@ -593,12 +594,13 @@ def re_average_z(args):
 
 
 def rebuild_optimisers(args):
-    """pixray.py:520-555: a FRESH Adam at learning_rate / 10^drops (or the drawer's own rate, fftdrawer.py:63-67)."""
+    """pixray.py:520-555: a FRESH args.optimiser at learning_rate / 10^drops, or the drawer's own Adam and rate
+    (fftdrawer.py:63-67)."""
     st = _state
     drop_divisor = 10 ** st.num_loss_drop
     own = st.drawer.get_opts(drop_divisor)
     st.lr = own[0]["lr"] if own else args.learning_rate / drop_divisor
-    st.engine.reset_optimizer()
+    P.install_optimiser(st.engine, "Adam" if own else args.optimiser)
     return st.lr
 
 
@@ -613,8 +615,8 @@ def checkdrop(args, it, losses):
 
 
 def train(args, cur_it):
-    """pixray.py:1436-1512.  The whole iteration (synth -> cutouts -> encode -> losses -> backward -> Adam -> clip_z) is
-    ONE pxr_iterate call.  Default: checkdrop, the scheduled learning-rate drops and auto-stop are decided inside that
+    """pixray.py:1436-1512.  The whole iteration (synth -> cutouts -> encode -> losses -> backward -> optimiser step ->
+    clip_z) is ONE pxr_iterate call.  Default: checkdrop, the scheduled learning-rate drops and auto-stop are decided inside that
     call on the device (pxr_set_schedule) and the host only POLLS a pinned status record -- no synchronisation in the
     loop; iterations enqueued after the device raised `stopped` leave z untouched, so the result equals the reference's
     control flow.  With b200_device_checkdrop=False (and for vdiff) the reference's host-side flow runs as written, one
@@ -639,11 +641,11 @@ def train(args, cur_it):
             did_drop = checkdrop(args, cur_it, st.losses)
             if args.auto_stop is True:
                 rebuild = did_drop
-    if isinstance(st.drawer, P.VdiffDrawer) and cur_it >= 1:  # pixray.py:1489-1495
+    if isinstance(st.drawer, P.VdiffDrawer) and cur_it >= 1:  # pixray.py:1489-1495: a fresh Adam whatever args.optimiser
         lr = float(st.drawer.sigmas[cur_it] / st.drawer.alphas[cur_it])
         st.drawer.makenoise(cur_it)
         st.lr = min(lr * 0.001, 0.01)
-        st.engine.reset_optimizer()
+        P.install_optimiser(st.engine, "Adam")
     if cur_it == args.iterations:
         checkin(args, cur_it, st.losses)
         return False

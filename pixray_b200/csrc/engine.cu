@@ -50,8 +50,10 @@ class Engine {
   // ---- drawer
   float* z_buf = nullptr;   // engine copy of z
   float* z_grad = nullptr;
-  float *adam_m = nullptr, *adam_v = nullptr;
-  int adam_t = 0;
+  float *adam_m = nullptr, *adam_v = nullptr;  // optimiser state s0 / s1 (kernels.cuh OptState)
+  float* opt_prev = nullptr;                   // s2: DiffGrad's previous gradient
+  int opt_kind = OPT_ADAM;                     // PXR_OPT_*
+  int adam_t = 0;                              // steps of the current optimiser instance
   // device-side checkdrop / learning-rate drops / auto-stop (kernels.cuh): off until pxr_set_schedule
   bool managed = false;
   DropConfig drop_cfg{};
@@ -638,6 +640,7 @@ class Engine {
   void step(float lr);
   void step_managed(int iter);
   void write_initial_drop_state();
+  void zero_optimizer_state();
 };
 
 Engine::~Engine() {
@@ -2171,8 +2174,8 @@ bool Engine::spot_pass(int which, bool accumulate_img) {
 void Engine::step(float lr) {
   ++adam_t;
   const int per_channel = (cfg.drawer == PXR_DRAWER_VQGAN) ? (int)(z_numel / cfg.z_channels) : 1;
-  adam_clip_step(z_buf, adam_m, adam_v, batches > 1 ? z_grad_acc : z_grad, 1.f, (int)z_numel, per_channel, zmin, zmax,
-                 cfg.drawer == PXR_DRAWER_PIXEL, lr, cfg.beta1, cfg.beta2, cfg.adam_eps, adam_t, st);
+  opt_clip_step(opt_kind, z_buf, OptState{adam_m, adam_v, opt_prev}, batches > 1 ? z_grad_acc : z_grad, 1.f, (int)z_numel,
+                per_channel, zmin, zmax, cfg.drawer == PXR_DRAWER_PIXEL, lr, cfg.beta1, cfg.beta2, cfg.adam_eps, adam_t, st);
   launches += 1;
 }
 
@@ -2331,13 +2334,19 @@ void Engine::write_initial_drop_state() {
   memset(const_cast<DropStatus*>(drop_status), 0, sizeof(DropStatus));
 }
 
+void Engine::zero_optimizer_state() {
+  PXR_CUDA(cudaMemsetAsync(adam_m, 0, z_numel * sizeof(float), st));
+  PXR_CUDA(cudaMemsetAsync(adam_v, 0, z_numel * sizeof(float), st));
+  PXR_CUDA(cudaMemsetAsync(opt_prev, 0, z_numel * sizeof(float), st));
+}
+
 // opt.step() + clip_z + checkdrop + (scheduled | auto-stop) optimiser rebuild, all decided on the device
 void Engine::step_managed(int iter) {
   const int per_channel = (cfg.drawer == PXR_DRAWER_VQGAN) ? (int)(z_numel / cfg.z_channels) : 1;
   const float* g = batches > 1 ? z_grad_acc : z_grad;
-  adam_clip_managed(z_buf, adam_m, adam_v, g, best_z, 1.f, (int)z_numel, per_channel, zmin, zmax,
-                    cfg.drawer == PXR_DRAWER_PIXEL, cfg.beta1, cfg.beta2, cfg.adam_eps, losses_dev, num_losses(), iter,
-                    drop_cfg, drop_state + drop_parity, drop_state + (drop_parity ^ 1), drop_status_dev, st);
+  opt_clip_managed(opt_kind, z_buf, OptState{adam_m, adam_v, opt_prev}, g, best_z, 1.f, (int)z_numel, per_channel, zmin,
+                   zmax, cfg.drawer == PXR_DRAWER_PIXEL, cfg.beta1, cfg.beta2, cfg.adam_eps, losses_dev, num_losses(), iter,
+                   drop_cfg, drop_state + drop_parity, drop_state + (drop_parity ^ 1), drop_status_dev, st);
   drop_parity ^= 1;
   launches += 1;
 }
@@ -2351,6 +2360,7 @@ void Engine::finalize() {
   else throw EngineError(-47, "unknown drawer kind");
   adam_m = dalloc<float>(z_numel);
   adam_v = dalloc<float>(z_numel);
+  opt_prev = dalloc<float>(z_numel);
   z_grad_acc = dalloc<float>(z_numel);
   best_z = dalloc<float>(z_numel);
   drop_state = dalloc<DropState>(2);
@@ -2814,8 +2824,7 @@ int pxr_set_schedule(pxr_handle h, float base_lr, int iter_drop_delay, int max_l
     e->drop_cfg.n_sched = n_drops;
     for (int i = 0; i < n_drops; ++i) e->drop_cfg.sched[i] = drops[i];
     e->managed = true;
-    PXR_CUDA(cudaMemsetAsync(e->adam_m, 0, e->z_numel * sizeof(float), e->st));
-    PXR_CUDA(cudaMemsetAsync(e->adam_v, 0, e->z_numel * sizeof(float), e->st));
+    e->zero_optimizer_state();
     e->write_initial_drop_state();
   });
 }
@@ -3123,30 +3132,44 @@ int pxr_read_losses(pxr_handle h, float* out_host) {
 int pxr_reset_optimizer(pxr_handle h) {
   PXR_TRY(h, {
     Engine* e = h->e;
-    PXR_CUDA(cudaMemsetAsync(e->adam_m, 0, e->z_numel * sizeof(float), e->st));
-    PXR_CUDA(cudaMemsetAsync(e->adam_v, 0, e->z_numel * sizeof(float), e->st));
+    e->zero_optimizer_state();
     e->adam_t = 0;
     if (e->managed) e->write_initial_drop_state();  // a fresh session: best-loss tracking and the drop count restart too
   });
 }
 
-// ---- checkpoint of the optimisation state (z, Adam m / v / step, the drop bookkeeping): resume = load + keep iterating
+int pxr_set_optimizer(pxr_handle h, int kind) {
+  if (kind < 0 || kind >= pxr::OPT_KINDS) {
+    h->e->err = "pxr_set_optimizer: unknown optimiser kind " + std::to_string(kind);
+    return -75;
+  }
+  h->e->opt_kind = kind;
+  return pxr_reset_optimizer(h);
+}
+
+// ---- checkpoint of the optimisation state (z, optimiser state / kind / step, the drop bookkeeping): resume = load + keep
+// iterating
 namespace {
 struct StateHeader {
   uint32_t magic, version;
   int64_t z_numel;
-  int32_t adam_t, managed, drop_parity, pad;
+  int32_t adam_t, managed, drop_parity;
+  int32_t opt_kind;  // PXR_OPT_*; 0 (Adam) in blobs written before the engine had other optimisers
   pxr::DropState drop;
 };
 constexpr uint32_t kStateMagic = 0x50585253u;  // "PXRS"
+const char* const kOptNames[pxr::OPT_KINDS] = {"Adam", "AdamW", "Adagrad", "Adamax", "DiffGrad"};
+// z, s0, s1, and s2 only for DiffGrad: an Adam blob keeps the size and layout it always had
+int state_buffers(int kind) { return kind == pxr::OPT_DIFFGRAD ? 4 : 3; }
+const char* opt_name(int kind) { return kind >= 0 && kind < pxr::OPT_KINDS ? kOptNames[kind] : "unknown"; }
 }  // namespace
 
 int pxr_state_size(pxr_handle h, int64_t* nbytes) {
-  *nbytes = (int64_t)sizeof(StateHeader) + 3 * h->e->z_numel * (int64_t)sizeof(float);
+  *nbytes = (int64_t)sizeof(StateHeader) + state_buffers(h->e->opt_kind) * h->e->z_numel * (int64_t)sizeof(float);
   return 0;
 }
 
-// host buffer of pxr_state_size bytes <- {header, z, m, v}.  Blocking.
+// host buffer of pxr_state_size bytes <- {header, z, s0, s1[, s2]}.  Blocking.
 int pxr_save_state(pxr_handle h, void* host_buf) {
   PXR_TRY(h, {
     Engine* e = h->e;
@@ -3158,6 +3181,7 @@ int pxr_save_state(pxr_handle h, void* host_buf) {
     hd.adam_t = e->adam_t;
     hd.managed = e->managed ? 1 : 0;
     hd.drop_parity = e->drop_parity;
+    hd.opt_kind = e->opt_kind;
     if (e->managed)
       PXR_CUDA(cudaMemcpyAsync(&hd.drop, e->drop_state + e->drop_parity, sizeof(pxr::DropState), cudaMemcpyDeviceToHost, e->st));
     char* out = static_cast<char*>(host_buf);
@@ -3165,13 +3189,15 @@ int pxr_save_state(pxr_handle h, void* host_buf) {
     PXR_CUDA(cudaMemcpyAsync(out + sizeof hd, e->z_buf, zb, cudaMemcpyDeviceToHost, e->st));
     PXR_CUDA(cudaMemcpyAsync(out + sizeof hd + zb, e->adam_m, zb, cudaMemcpyDeviceToHost, e->st));
     PXR_CUDA(cudaMemcpyAsync(out + sizeof hd + 2 * zb, e->adam_v, zb, cudaMemcpyDeviceToHost, e->st));
+    if (state_buffers(e->opt_kind) > 3)
+      PXR_CUDA(cudaMemcpyAsync(out + sizeof hd + 3 * zb, e->opt_prev, zb, cudaMemcpyDeviceToHost, e->st));
     PXR_CUDA(cudaStreamSynchronize(e->st));
     memcpy(out, &hd, sizeof hd);
   });
 }
 
-// The inverse: the engine's z, Adam state and (when it was saved in managed mode and pxr_set_schedule was called here
-// too) the learning-rate / best-loss / drop-count bookkeeping.  Blocking.
+// The inverse: the engine's z, optimiser state (the blob's optimiser kind must be the engine's) and (when it was saved in
+// managed mode and pxr_set_schedule was called here too) the learning-rate / best-loss / drop-count bookkeeping.  Blocking.
 int pxr_load_state(pxr_handle h, const void* host_buf) {
   PXR_TRY(h, {
     Engine* e = h->e;
@@ -3180,11 +3206,16 @@ int pxr_load_state(pxr_handle h, const void* host_buf) {
     memcpy(&hd, host_buf, sizeof hd);
     if (hd.magic != kStateMagic || hd.version != 1) throw EngineError(-68, "pxr_load_state: not a pixray_b200 state blob");
     if (hd.z_numel != e->z_numel) throw EngineError(-68, "pxr_load_state: the blob belongs to a different latent shape");
+    if (hd.opt_kind != e->opt_kind)
+      throw EngineError(-68, std::string("pxr_load_state: the blob holds ") + opt_name(hd.opt_kind) +
+                                 " state but the engine's optimiser is " + opt_name(e->opt_kind) + " (pxr_set_optimizer first)");
     const char* in = static_cast<const char*>(host_buf);
     const size_t zb = (size_t)e->z_numel * sizeof(float);
     PXR_CUDA(cudaMemcpyAsync(e->z_buf, in + sizeof hd, zb, cudaMemcpyHostToDevice, e->st));
     PXR_CUDA(cudaMemcpyAsync(e->adam_m, in + sizeof hd + zb, zb, cudaMemcpyHostToDevice, e->st));
     PXR_CUDA(cudaMemcpyAsync(e->adam_v, in + sizeof hd + 2 * zb, zb, cudaMemcpyHostToDevice, e->st));
+    if (state_buffers(e->opt_kind) > 3)
+      PXR_CUDA(cudaMemcpyAsync(e->opt_prev, in + sizeof hd + 3 * zb, zb, cudaMemcpyHostToDevice, e->st));
     e->adam_t = hd.adam_t;
     if (hd.managed && e->managed) {
       PXR_CUDA(cudaMemcpyAsync(e->drop_state + e->drop_parity, &hd.drop, sizeof(pxr::DropState), cudaMemcpyHostToDevice, e->st));

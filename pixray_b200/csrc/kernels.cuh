@@ -207,27 +207,55 @@ void prompt_loss(const float* e, int B, int D, const float* prompts, const float
                  const int* slots, const float* inv_rows, int n, int cutn_global, float grad_scale, float* e_unit,
                  float* losses, float* de, act_t* de16, cudaStream_t st);
 
-// ------------------------------------------------------------------ optimiser (pixray.py:538-539, 1484-1487)
-// Adam (bias-corrected, torch.optim.Adam semantics) on z with gradient g * inv_scale, then clip_z to per-channel
-// [zmin, zmax] (vqgan.py:202-204) or [0,1] when zmin == nullptr && clip01.
-void adam_clip_step(float* z, float* m, float* v, const float* g, float inv_scale, int n, int per_channel,
-                    const float* zmin, const float* zmax, int clip01, float lr, float b1, float b2, float eps, int t,
-                    cudaStream_t st);
+// ------------------------------------------------------------------ optimiser (pixray.py:520-555, 1484-1487)
+// The optimisers rebuild_optimisers can build (`--optimiser`), with the library defaults (the reference passes only lr):
+// torch.optim.Adam, AdamW (weight decay 0.01), Adagrad (eps 1e-10, lr_decay 0, initial accumulator 0), Adamax, and
+// torch_optimizer.DiffGrad 0.1.0.  Betas / eps of the Adam family come from pxr_config (defaults 0.9 / 0.999 / 1e-8).
+// Values are the PXR_OPT_* of the C ABI.
+enum OptKind { OPT_ADAM = 0, OPT_ADAMW = 1, OPT_ADAGRAD = 2, OPT_ADAMAX = 3, OPT_DIFFGRAD = 4 };
+constexpr int OPT_KINDS = 5;
+constexpr float ADAMW_WEIGHT_DECAY = 0.01f;
+// Per-element state, z_numel floats each.  s0: first moment (Adam, AdamW, Adamax, DiffGrad); s1: second moment (Adam,
+// AdamW, DiffGrad), sum of squared gradients (Adagrad) or infinity norm (Adamax); s2: previous gradient (DiffGrad).
+struct OptState {
+  float *s0, *s1, *s2;
+};
+// The step's scalars, from the learning rate and the step count t of the current optimiser instance (1-based).
+struct OptCoef {
+  float step_size;     // Adam / AdamW / Adamax: lr / (1 - b1^t); Adagrad: lr; DiffGrad: lr sqrt(1 - b2^t) / (1 - b1^t)
+  float inv_sqrt_bc2;  // Adam / AdamW: 1 / sqrt(1 - b2^t)
+  float decay;         // AdamW: 1 - lr * weight_decay, applied to z before the step
+};
+__host__ __device__ inline OptCoef opt_coef(int kind, float lr, float b1, float b2, int t) {
+  const double bc1 = 1.0 - pow((double)b1, (double)t), bc2 = 1.0 - pow((double)b2, (double)t);
+  OptCoef c;
+  c.step_size = (float)((double)lr / bc1);
+  c.inv_sqrt_bc2 = (float)(1.0 / sqrt(bc2));
+  c.decay = kind == OPT_ADAMW ? (float)(1.0 - (double)lr * (double)ADAMW_WEIGHT_DECAY) : 1.f;
+  if (kind == OPT_ADAGRAD) c.step_size = lr;
+  if (kind == OPT_DIFFGRAD) c.step_size = (float)((double)lr * sqrt(bc2) / bc1);
+  return c;
+}
+// One step of optimiser `kind` on z with gradient g * inv_scale (t = its step count, 1-based), then clip_z to
+// per-channel [zmin, zmax] (vqgan.py:202-204) or [0,1] when zmin == nullptr && clip01.
+void opt_clip_step(int kind, float* z, OptState s, const float* g, float inv_scale, int n, int per_channel,
+                   const float* zmin, const float* zmax, int clip01, float lr, float b1, float b2, float eps, int t,
+                   cudaStream_t st);
 
-// ------------------------------------------------------------------ device-side checkdrop + Adam (pixray.py:1090-1109, 1464-1512)
+// ------------------------------------------------------------------ device-side checkdrop + optimiser step (pixray.py:1090-1109, 1464-1512)
 // train()'s per-iteration control decisions without a host round trip.  The optimiser step of iteration `it` reads the
-// iteration's loss vector, decides like checkdrop / the scheduled learning-rate drops / auto_stop do, applies Adam + clip_z
-// with the CURRENT learning rate and Adam state, and -- when the decision is "rebuild the optimisers" -- leaves a fresh
-// Adam (m = v = 0, t = 0) at learning_rate / 10^num_loss_drop behind for the next iteration, or raises `stopped` when
-// the drops are used up (after which further iterations leave z untouched).  State is double-buffered (read cur, write
-// next) so every block of the kernel sees the same decision inputs.
+// iteration's loss vector, decides like checkdrop / the scheduled learning-rate drops / auto_stop do, applies the step +
+// clip_z with the CURRENT learning rate and optimiser state, and -- when the decision is "rebuild the optimisers" --
+// leaves a fresh optimiser of the same kind (state zeroed, t = 0) at learning_rate / 10^num_loss_drop behind for the next
+// iteration, or raises `stopped` when the drops are used up (after which further iterations leave z untouched).  State
+// is double-buffered (read cur, write next) so every block of the kernel sees the same decision inputs.
 struct DropState {
   float best_loss;     // 1e20 after a rebuild (pixray.py:1509)
   int best_iter;
   int num_loss_drop;
   int stopped;
   float lr;
-  int adam_t;          // steps taken by the current Adam instance
+  int adam_t;          // steps taken by the current optimiser instance (whichever kind)
   int pad[2];
 };
 struct DropConfig {
@@ -250,10 +278,10 @@ struct DropStatus {
   float losses[64];
   volatile int seq_end;
 };
-void adam_clip_managed(float* z, float* m, float* v, const float* g, float* best_z, float inv_scale, int n,
-                       int per_channel, const float* zmin, const float* zmax, int clip01, float b1, float b2,
-                       float eps, const float* losses, int n_losses, int iter, const DropConfig& cfg,
-                       const DropState* cur, DropState* next, DropStatus* status_mapped, cudaStream_t st);
+void opt_clip_managed(int kind, float* z, OptState s, const float* g, float* best_z, float inv_scale, int n,
+                      int per_channel, const float* zmin, const float* zmax, int clip01, float b1, float b2, float eps,
+                      const float* losses, int n_losses, int iter, const DropConfig& cfg, const DropState* cur,
+                      DropState* next, DropStatus* status_mapped, cudaStream_t st);
 // acc (=|+=) g: gradient accumulation over the `batches` passes of one iteration (pixray.py:1464-1482)
 void accumulate_f32(const float* g, float* acc, long long n, int accumulate, cudaStream_t st);
 

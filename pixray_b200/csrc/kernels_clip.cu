@@ -1,9 +1,10 @@
 // CLIP-side row kernels: LayerNorm fwd/bwd on the fp32 residual stream, attention softmax fwd/bwd, the
-// class-token head (ln_post + proj), the Prompt / spherical-distance loss with its gradient, Adam + clip_z.
+// class-token head (ln_post + proj), the Prompt / spherical-distance loss with its gradient, the optimiser step + clip_z.
 #include "kernels.cuh"
 #include "launch.cuh"
 #include <cfloat>
 #include <cmath>
+#include <stdexcept>
 
 namespace pxr {
 namespace {
@@ -461,66 +462,116 @@ __global__ void __launch_bounds__(128) prompt_loss_kernel(const float* __restric
   }
 }
 
-__global__ void adam_clip_kernel(float* __restrict__ z, float* __restrict__ m, float* __restrict__ v,
-                                 const float* __restrict__ g, float inv_scale, int n, int per_channel,
-                                 const float* __restrict__ zmin, const float* __restrict__ zmax, int clip01,
-                                 float step_size, float b1, float b2, float eps, float inv_sqrt_bc2) {
+// clip_z after the optimiser step: per-channel [zmin, zmax] (vqgan.py:202-204) or [0, 1] (fast_pixeldrawer.py:98-100)
+__device__ __forceinline__ float clip_z_one(float zi, int i, int per_channel, const float* __restrict__ zmin,
+                                            const float* __restrict__ zmax, int clip01) {
+  if (zmin) {
+    const int c = i / per_channel;
+    zi = fminf(fmaxf(zi, zmin[c]), zmax[c]);
+  } else if (clip01) {
+    zi = fminf(fmaxf(zi, 0.f), 1.f);
+  }
+  return zi;
+}
+
+// Adam's moments: m = b1 m + (1 - b1) g, v = b2 v + (1 - b2) g^2, rounded as fma(b1, m, (1 - b1) g) and
+// fma(b2, v, ((1 - b2) g) g)
+__device__ __forceinline__ float adam_m(float m, float g, float b1) { return __fmaf_rn(b1, m, __fmul_rn(1.f - b1, g)); }
+__device__ __forceinline__ float adam_v(float v, float g, float b2) {
+  return __fmaf_rn(b2, v, __fmul_rn(__fmul_rn(1.f - b2, g), g));
+}
+
+// One optimiser step on element i (see kernels.cuh "optimiser").  Returns the new z (before clip_z) and writes the
+// updated state, or zeroes it when `fresh` (the managed kernel's rebuild: the NEXT step starts from a new optimiser).
+template <int K>
+__device__ __forceinline__ float opt_update(float zi, float gi, const OptState& s, int i, float b1, float b2, float eps,
+                                            const OptCoef& c, bool fresh) {
+  if constexpr (K == OPT_ADAM || K == OPT_ADAMW) {
+    if constexpr (K == OPT_ADAMW) zi = zi * c.decay;  // torch.optim.AdamW: decoupled decay BEFORE the Adam step
+    // torch.optim.Adam: step_size = lr / (1 - b1^t); denom = sqrt(v) / sqrt(1 - b2^t) + eps.  The roundings are pinned
+    // so that every instantiation keeps the contraction the Adam-only kernels had (same bits as before).
+    const float mi = adam_m(s.s0[i], gi, b1);
+    const float vi = adam_v(s.s1[i], gi, b2);
+    s.s0[i] = fresh ? 0.f : mi;
+    s.s1[i] = fresh ? 0.f : vi;
+    const float denom = __fmaf_rn(sqrtf(vi), c.inv_sqrt_bc2, eps);
+    return zi - __fmul_rn(c.step_size, mi) / denom;
+  } else if constexpr (K == OPT_ADAGRAD) {
+    // torch.optim.Adagrad (lr_decay 0, initial accumulator 0): sum += g^2; z -= lr * g / (sqrt(sum) + 1e-10)
+    const float si = s.s1[i] + gi * gi;
+    s.s1[i] = fresh ? 0.f : si;
+    return zi - c.step_size * (gi / (sqrtf(si) + 1e-10f));
+  } else if constexpr (K == OPT_ADAMAX) {
+    // torch.optim.Adamax: m.lerp_(g, 1 - b1); u = max(b2 u, |g| + eps); z -= lr / (1 - b1^t) * m / u
+    const float m0 = s.s0[i];
+    const float mi = m0 + (1.f - b1) * (gi - m0);
+    const float ui = fmaxf(b2 * s.s1[i], fabsf(gi) + eps);
+    s.s0[i] = fresh ? 0.f : mi;
+    s.s1[i] = fresh ? 0.f : ui;
+    return zi - c.step_size * (mi / ui);
+  } else {
+    static_assert(K == OPT_DIFFGRAD, "unknown optimiser kind");
+    // torch_optimizer.DiffGrad 0.1.0: m, v as Adam; denom = sqrt(v) + eps (eps NOT bias-corrected);
+    // dfc = 1 / (1 + exp(-|p - g|)); p = g; z -= lr sqrt(1 - b2^t) / (1 - b1^t) * (m dfc) / denom
+    const float mi = adam_m(s.s0[i], gi, b1);
+    const float vi = adam_v(s.s1[i], gi, b2);
+    const float dfc = 1.f / (1.f + expf(-fabsf(s.s2[i] - gi)));
+    s.s0[i] = fresh ? 0.f : mi;
+    s.s1[i] = fresh ? 0.f : vi;
+    s.s2[i] = fresh ? 0.f : gi;
+    const float denom = sqrtf(vi) + eps;
+    return zi - c.step_size * ((mi * dfc) / denom);
+  }
+}
+
+template <int K>
+__global__ void opt_clip_kernel(float* __restrict__ z, OptState s, const float* __restrict__ g, float inv_scale, int n,
+                                int per_channel, const float* __restrict__ zmin, const float* __restrict__ zmax,
+                                int clip01, float b1, float b2, float eps, OptCoef c) {
   pdl_prologue();
   int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  float gi = g[i] * inv_scale;
-  float mi = b1 * m[i] + (1.f - b1) * gi;
-  float vi = b2 * v[i] + (1.f - b2) * gi * gi;
-  m[i] = mi;
-  v[i] = vi;
-  float denom = sqrtf(vi) * inv_sqrt_bc2 + eps;
-  float zi = z[i] - step_size * mi / denom;
-  if (zmin) {
-    int c = i / per_channel;
-    zi = fminf(fmaxf(zi, zmin[c]), zmax[c]);  // vqgan.py:202-204
-  } else if (clip01) {
-    zi = fminf(fmaxf(zi, 0.f), 1.f);  // fast_pixeldrawer.py:98-100
-  }
-  z[i] = zi;
+  const float gi = g[i] * inv_scale;
+  const float zi = opt_update<K>(z[i], gi, s, i, b1, b2, eps, c, false);
+  z[i] = clip_z_one(zi, i, per_channel, zmin, zmax, clip01);
 }
 
-// see kernels.cuh "device-side checkdrop + Adam"
-__global__ void adam_clip_managed_kernel(float* __restrict__ z, float* __restrict__ m, float* __restrict__ v,
-                                         const float* __restrict__ g, float* __restrict__ best_z, float inv_scale, int n,
-                                         int per_channel, const float* __restrict__ zmin, const float* __restrict__ zmax,
-                                         int clip01, float b1, float b2, float eps, const float* __restrict__ losses,
-                                         int n_losses, int iter, DropConfig cfg, const DropState* __restrict__ cur,
-                                         DropState* __restrict__ next, DropStatus* status) {
+// see kernels.cuh "device-side checkdrop + optimiser step"
+template <int K>
+__global__ void opt_clip_managed_kernel(float* __restrict__ z, OptState s, const float* __restrict__ g,
+                                        float* __restrict__ best_z, float inv_scale, int n, int per_channel,
+                                        const float* __restrict__ zmin, const float* __restrict__ zmax, int clip01,
+                                        float b1, float b2, float eps, const float* __restrict__ losses, int n_losses,
+                                        int iter, DropConfig cfg, const DropState* __restrict__ cur,
+                                        DropState* __restrict__ next, DropStatus* status) {
   pdl_prologue();
-  const DropState s = *cur;
+  const DropState ds = *cur;
   const bool writer = blockIdx.x == 0 && threadIdx.x == 0;
   float loss_sum = 0.f;
   for (int k = 0; k < n_losses; ++k) loss_sum += losses[k];  // sum(lossAll): left to right in fp32 like Python's sum()
-  DropState nx = s;
+  DropState nx = ds;
   bool rebuild = false, new_best = false;
-  if (!s.stopped) {
+  if (!ds.stopped) {
     bool scheduled = false;
     for (int k = 0; k < cfg.n_sched; ++k) scheduled |= (cfg.sched[k] == iter);
     if (scheduled) {
       rebuild = true;  // "Dropping learning rate" (pixray.py:1468-1470): checkdrop is not consulted on these iterations
     } else {
       bool drop = false;
-      if (loss_sum < s.best_loss) {
+      if (loss_sum < ds.best_loss) {
         new_best = true;
         nx.best_loss = loss_sum;
         nx.best_iter = iter;
-      } else if (iter - s.best_iter >= cfg.iter_drop_delay) {
+      } else if (iter - ds.best_iter >= cfg.iter_drop_delay) {
         drop = true;
       }
       if (cfg.auto_stop) rebuild = drop;
     }
-    const int t = s.adam_t + 1;
+    const int t = ds.adam_t + 1;
     nx.adam_t = t;
-    // torch.optim.Adam: step_size = lr / (1 - b1^t); denom = sqrt(v) / sqrt(1 - b2^t) + eps
-    const double bc1 = 1.0 - pow((double)b1, (double)t), bc2 = 1.0 - pow((double)b2, (double)t);
-    const float step_size = (float)((double)s.lr / bc1), inv_sqrt_bc2 = (float)(1.0 / sqrt(bc2));
+    const OptCoef c = opt_coef(K, ds.lr, b1, b2, t);
     if (rebuild) {
-      nx.num_loss_drop = s.num_loss_drop + 1;
+      nx.num_loss_drop = ds.num_loss_drop + 1;
       if (nx.num_loss_drop > cfg.max_loss_drops) {
         nx.stopped = 1;  // train() returns False (pixray.py:1505-1506); this iteration's step still happened
       } else {
@@ -535,19 +586,8 @@ __global__ void adam_clip_managed_kernel(float* __restrict__ z, float* __restric
       const float z0 = z[i];
       if (new_best && best_z) best_z[i] = z0;  // best_z = drawer.get_z_copy() (pixray.py:1104): z BEFORE this step
       const float gi = g[i] * inv_scale;
-      const float mi = b1 * m[i] + (1.f - b1) * gi;
-      const float vi = b2 * v[i] + (1.f - b2) * gi * gi;
-      m[i] = fresh ? 0.f : mi;
-      v[i] = fresh ? 0.f : vi;
-      const float denom = sqrtf(vi) * inv_sqrt_bc2 + eps;
-      float zi = z0 - step_size * mi / denom;
-      if (zmin) {
-        const int c = i / per_channel;
-        zi = fminf(fmaxf(zi, zmin[c]), zmax[c]);
-      } else if (clip01) {
-        zi = fminf(fmaxf(zi, 0.f), 1.f);
-      }
-      z[i] = zi;
+      const float zi = opt_update<K>(z0, gi, s, i, b1, b2, eps, c, fresh);
+      z[i] = clip_z_one(zi, i, per_channel, zmin, zmax, clip01);
     }
   }
   if (writer) {
@@ -671,23 +711,32 @@ void prompt_loss(const float* e, int B, int D, const float* prompts, const float
                                                            1.f / cutn_global, grad_scale, e_unit, losses, de, de16);
 }
 
-void adam_clip_step(float* z, float* m, float* v, const float* g, float inv_scale, int n, int per_channel,
-                    const float* zmin, const float* zmax, int clip01, float lr, float b1, float b2, float eps, int t,
-                    cudaStream_t st) {
-  // torch.optim.Adam: step_size = lr / (1 - b1^t); denom = sqrt(v) / sqrt(1 - b2^t) + eps
-  const double bc1 = 1.0 - pow((double)b1, t), bc2 = 1.0 - pow((double)b2, t);
-  launch_pdl(adam_clip_kernel, dim3((n + 255) / 256), dim3(256), 0, st, z, m, v, g, inv_scale, n, per_channel, zmin, zmax, clip01,
-                                                    (float)(lr / bc1), b1, b2, eps, (float)(1.0 / sqrt(bc2)));
+#define OPT_DISPATCH(KERNEL, GRID, ...)                                                                 \
+  switch (kind) {                                                                                       \
+    case OPT_ADAM: launch_pdl(KERNEL<OPT_ADAM>, GRID, dim3(256), 0, st, __VA_ARGS__); break;            \
+    case OPT_ADAMW: launch_pdl(KERNEL<OPT_ADAMW>, GRID, dim3(256), 0, st, __VA_ARGS__); break;          \
+    case OPT_ADAGRAD: launch_pdl(KERNEL<OPT_ADAGRAD>, GRID, dim3(256), 0, st, __VA_ARGS__); break;      \
+    case OPT_ADAMAX: launch_pdl(KERNEL<OPT_ADAMAX>, GRID, dim3(256), 0, st, __VA_ARGS__); break;        \
+    case OPT_DIFFGRAD: launch_pdl(KERNEL<OPT_DIFFGRAD>, GRID, dim3(256), 0, st, __VA_ARGS__); break;    \
+    default: throw std::runtime_error("unknown optimiser kind");                                        \
+  }
+
+void opt_clip_step(int kind, float* z, OptState s, const float* g, float inv_scale, int n, int per_channel,
+                   const float* zmin, const float* zmax, int clip01, float lr, float b1, float b2, float eps, int t,
+                   cudaStream_t st) {
+  const OptCoef c = opt_coef(kind, lr, b1, b2, t);
+  OPT_DISPATCH(opt_clip_kernel, dim3((n + 255) / 256), z, s, g, inv_scale, n, per_channel, zmin, zmax, clip01, b1, b2,
+               eps, c)
 }
 
-void adam_clip_managed(float* z, float* m, float* v, const float* g, float* best_z, float inv_scale, int n,
-                       int per_channel, const float* zmin, const float* zmax, int clip01, float b1, float b2,
-                       float eps, const float* losses, int n_losses, int iter, const DropConfig& cfg,
-                       const DropState* cur, DropState* next, DropStatus* status_mapped, cudaStream_t st) {
+void opt_clip_managed(int kind, float* z, OptState s, const float* g, float* best_z, float inv_scale, int n,
+                      int per_channel, const float* zmin, const float* zmax, int clip01, float b1, float b2, float eps,
+                      const float* losses, int n_losses, int iter, const DropConfig& cfg, const DropState* cur,
+                      DropState* next, DropStatus* status_mapped, cudaStream_t st) {
   int grid = (n + 255) / 256;
   if (grid > 148 * 4) grid = 148 * 4;
-  launch_pdl(adam_clip_managed_kernel, dim3(grid), dim3(256), 0, st, z, m, v, g, best_z, inv_scale, n, per_channel, zmin,
-             zmax, clip01, b1, b2, eps, losses, n_losses, iter, cfg, cur, next, status_mapped);
+  OPT_DISPATCH(opt_clip_managed_kernel, dim3(grid), z, s, g, best_z, inv_scale, n, per_channel, zmin, zmax, clip01, b1,
+               b2, eps, losses, n_losses, iter, cfg, cur, next, status_mapped)
 }
 
 void accumulate_f32(const float* g, float* acc, long long n, int accumulate, cudaStream_t st) {

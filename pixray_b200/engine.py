@@ -16,6 +16,8 @@ ANCHOR_SPHERICAL, ANCHOR_MSE, ANCHOR_COS, ANCHOR_PIX = 0, 1, 2, 3
 FILTER_TILER, FILTER_WALLPAPER, FILTER_LOOKUP = range(3)
 PAD_REFLECTION, PAD_BORDER = 0, 1
 MOD_VQGAN, MOD_CLIP0, MOD_CLIP1 = 0, 1, 2
+# args.optimiser (pixray.py:536-553) -> PXR_OPT_*; each with its library's defaults, only lr is set
+OPTIMISERS = {"Adam": 0, "AdamW": 1, "Adagrad": 2, "Adamax": 3, "DiffGrad": 4}
 
 VQGAN_F16_16384 = dict(z_channels=256, n_embed=16384, ch=128, ch_mult=(1, 1, 2, 2, 4), num_res_blocks=2,
                        attn_resolution=16, resolution=256)
@@ -90,6 +92,7 @@ class B200Engine:
         self.h = h
         self._keep = []
         self._ext = None  # torch view of the engine's stream (ordering against torch-side producers of z / noise)
+        self.optimizer = "Adam"  # the kind pxr_create starts with; set_optimizer changes it
 
     # ------------------------------------------------------------------ plumbing
     def _check(self, rc, what):
@@ -403,10 +406,18 @@ class B200Engine:
         return z
 
     def reset_optimizer(self):
+        """A fresh instance of the current optimiser: state zeroed, step count 0 (pxr_reset_optimizer)."""
         self._check(self.lib.pxr_reset_optimizer(self.h), "pxr_reset_optimizer")
 
+    def set_optimizer(self, name):
+        """Switch to the optimiser `name` (a key of OPTIMISERS) with fresh state (pxr_set_optimizer)."""
+        if name not in OPTIMISERS:
+            raise NotImplementedError(f"optimiser '{name}' is not built; available: {sorted(OPTIMISERS)}")
+        self._check(self.lib.pxr_set_optimizer(self.h, OPTIMISERS[name]), "pxr_set_optimizer")
+        self.optimizer = name
+
     def save_state(self):
-        """bytes: z, Adam m / v / step and the drop bookkeeping (pxr_save_state)."""
+        """bytes: z, the optimiser's state / kind / step and the drop bookkeeping (pxr_save_state)."""
         n = C.c_int64()
         self.lib.pxr_state_size(self.h, C.byref(n))
         buf = (C.c_ubyte * n.value)()

@@ -441,12 +441,22 @@ def parse_prompt(prompt):
 from .util import get_learning_rate_drops  # noqa: E402,F401  (pixray.py:1999-2003)
 
 
-class Optimizer:
-    """optim.Adam([drawer.get_z()], lr) as rebuild_optimisers builds it (pixray.py:520-555): zero_grad / step."""
+def install_optimiser(engine, name):
+    """A fresh optimiser `name` (Adam, AdamW, Adagrad, Adamax or DiffGrad) on the engine.  The engine switches kind only
+    when `name` differs from its current one; otherwise this is a plain reset of the current optimiser's state."""
+    if name != getattr(engine, "optimizer", "Adam"):
+        engine.set_optimizer(name)
+    else:
+        engine.reset_optimizer()
 
-    def __init__(self, session: Session, drawer, lr):
+
+class Optimizer:
+    """optim.<optimiser>([drawer.get_z()], lr) as rebuild_optimisers builds it (pixray.py:520-555): zero_grad / step.
+    optimiser: Adam, AdamW, Adagrad, Adamax or DiffGrad, each with its library's defaults."""
+
+    def __init__(self, session: Session, drawer, lr, optimiser="Adam"):
         self.session, self.drawer, self.lr = session, drawer, lr
-        session.engine.reset_optimizer()
+        install_optimiser(session.engine, optimiser)
 
     def zero_grad(self):
         z = self.drawer.get_z()
@@ -475,10 +485,11 @@ def train_iteration(session: Session, drawer, make_cutouts, perceptors, prompt_t
     opt.step()
     drawer.clip_z()
     if isinstance(drawer, VdiffDrawer) and session.cur_iteration >= 1:
-        # pixray.py:1489-1495: re-noise x for the next timestep and start a fresh Adam with the schedule's step size
+        # pixray.py:1489-1495: re-noise x for the next timestep and start a fresh Adam (whatever the optimiser setting)
+        # with the schedule's step size
         it = session.cur_iteration
         lr = float(drawer.sigmas[it] / drawer.alphas[it])
         drawer.makenoise(it)
         opt.lr = min(lr * 0.001, 0.01)
-        session.engine.reset_optimizer()
+        install_optimiser(session.engine, "Adam")
     return result
